@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark: assembly Mbp polished / second (BASELINE.json).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One step = one pass of the polish hot path (classify -> CIGAR walk + pileup -> vote + compaction) over one
 synthetic workload (default: BASELINE configs[1], one 5 Mbp contig at 100x, multi-mapped 150 bp pairs).
@@ -16,6 +16,10 @@ With N > 1 (torchrun, one rank per GPU) the contigs of ONE config-5-shaped assem
 families that cross contigs) shard across the ranks with no collective on the data path: every rank polishes its
 shard, ghost records included (weak scaling); time = max over ranks.
 --impl reference times the reference's CPU path (the oracle; the Rust reference cannot be built here) on rank 0.
+K steps are timed on the kernel path and K on the e2e path.  The inputs are generated from fixed seeds, so they are the
+same from run to run.
+--dump-outputs DIR writes what the last timed step returned (rank 0's shard when N > 1) as DIR/<name>.npy, so that two
+builds can be compared output for output; that step also copies its result to the host, outside the device-timed stages.
 """
 import argparse
 import json
@@ -75,6 +79,7 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": []}
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, reasons = [], None, set()
         for s in self.samples:
             f = [x.strip() for x in s.split(",")]
@@ -127,6 +132,42 @@ def reference_sample(workload):
     return 1, clen, (depth if clen * depth <= 6e8 else 100.0), False
 
 
+DUMP_MAX_BYTES = 64_000_000
+DUMP_FULL_BASES = 12_000_000        # up to this many polished bases are written whole (48 MB as float32)
+DUMP_SAMPLE_BASES = 4_000_000       # above it, this many positions drawn with seed 0, and the positions (16 + 32 MB)
+
+
+def dump_outputs(out_dir, sequences, changed, zero_depth, total_depth, n_aln_used):
+    """Writes one polish result, as a caller of the polish call receives it, as float .npy files under out_dir:
+    polished_bases (the ASCII codes of the polished contigs, concatenated), contig_offsets (where each contig starts in
+    them, plus the total), changed, zero_depth and total_depth (per contig) and n_aln_used.  A result of more than
+    DUMP_FULL_BASES bases is sampled at DUMP_SAMPLE_BASES fixed positions, written as polished_bases_index.
+    All but total_depth are exact; the device sums total_depth in parallel, so it can differ in the last bits from run to
+    run (include/pp_abi.h).  Returns the names written."""
+    import numpy as np
+    bases = np.frombuffer(b"".join(sequences), dtype=np.uint8)
+    out = {"contig_offsets": np.cumsum([0] + [len(s) for s in sequences], dtype=np.int64).astype(np.float64),
+           "changed": np.asarray(changed, dtype=np.float64), "zero_depth": np.asarray(zero_depth, dtype=np.float64),
+           "total_depth": np.asarray(total_depth, dtype=np.float64), "n_aln_used": np.array([n_aln_used], dtype=np.float64)}
+    if bases.size <= DUMP_FULL_BASES:
+        out["polished_bases"] = bases.astype(np.float32)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(bases.size, DUMP_SAMPLE_BASES, replace=False))
+        out["polished_bases"] = bases[idx].astype(np.float32)
+        out["polished_bases_index"] = idx.astype(np.float64)
+    if sum(a.nbytes for a in out.values()) > DUMP_MAX_BYTES:
+        raise RuntimeError("bench: --dump-outputs would write more than %d bytes" % DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(out)
+
+
+def fasta_sequences(fasta):
+    """The sequence lines of a polished FASTA (one header line and one sequence line per contig)."""
+    return fasta.split(b"\n")[1::2]
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's own CPU implementation of the path on the host cores.  The Rust crate
     cannot be built in this image (no cargo/rustc; 78 un-vendored crates), so this is the oracle port, one thread (the
@@ -151,6 +192,8 @@ def run_reference(args, rank, world):
             sha = hashlib.sha256(r["fasta"]).hexdigest()
             if i >= args.warmup:
                 vals.append((bp / 1e6 / dt, dt, r["secs"]))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, fasta_sequences(r["fasta"]), r["changed"], r["zero_depth"], r["total_depth"], r["used_total"])
     finally:
         shutil.rmtree(d, ignore_errors=True)
     v = sum(x[0] for x in vals) / len(vals)
@@ -176,7 +219,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--wire4", action="store_true", help="e2e with the 4-bit arrays on the wire instead of the 2-bit format")
     ap.add_argument("--no-t3", action="store_true", help="skip the SAM-text-on-disk -> FASTA measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -283,8 +329,9 @@ def main():
     stage = {}
     dev_ms = 0.0
     launches = 0
-    for _ in range(args.steps):
-        r = ctx.polish_resident(fetch=False)
+    dump = bool(args.dump_outputs) and rank == 0
+    for i in range(args.steps):
+        r = ctx.polish_resident(fetch=dump and i == args.steps - 1)
         dev_ms += r["timing"]["total_ms"]
         launches += r["timing"]["launches"]
         for k, v in r["timing"].items():
@@ -294,6 +341,8 @@ def main():
     wall_ms = (time.perf_counter() - t0) * 1e3
     out_len = r["out_len"]
     ms_step = dev_ms / args.steps
+    if dump:
+        dump_outputs(args.dump_outputs, r["sequences"], r["changed"], r["zero_depth"], r["total_depth"], r["n_aln_used"])
 
     # ---------------- e2e: host buffers through pp_polish ----------------
     # (inputs in pinned host arrays, the result into caller-owned pinned buffers; the last result is checked against the
@@ -303,7 +352,7 @@ def main():
         e = ctx.polish_packed(cview, hv, into=out_res)
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     e2e_each = []
     for _ in range(e2e_steps):
         t1 = time.perf_counter()
@@ -464,4 +513,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
     main()
