@@ -151,60 +151,109 @@ static void mark(const char* what) {
     if (on) fprintf(stderr, "[timing] %8.1f ms  %s\n", std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(), what);
 }
 
+// The value after the option at tok[i] (which then points at the value).
+static const char* need(const std::vector<Token>& tok, size_t& i, const char* flag) {
+    if (i + 1 >= tok.size()) usage_error(std::string("a value is required for '") + flag + "' but none was supplied");
+    return tok[++i].text.c_str();
+}
+
+// The options of `polish` (except --debug and --gpus), `filter` and the additive ones every command takes.  Each parser takes the
+// option at tok[i] (and its value) and says whether it was one of its options.
+struct FilterArgs { std::string in1, in2, out1, out2, orientation = "auto"; double low = 0.1, high = 99.9; };
+struct CommonArgs { int device = 0; bool quiet = false, host_parse = false; };
+
+static bool polish_option(const std::vector<Token>& tok, size_t& i, pp_polish_params& prm) {
+    const std::string& a = tok[i].text;
+    if (a == "-i" || a == "--fraction_invalid") prm.fraction_invalid = parse_f64("--fraction_invalid <FRACTION_INVALID>", need(tok, i, "--fraction_invalid"));
+    else if (a == "-v" || a == "--fraction_valid") prm.fraction_valid = parse_f64("--fraction_valid <FRACTION_VALID>", need(tok, i, "--fraction_valid"));
+    else if (a == "-m" || a == "--max_errors") prm.max_errors = parse_u32("--max_errors <MAX_ERRORS>", need(tok, i, "--max_errors"));
+    else if (a == "-d" || a == "--min_depth") prm.min_depth = parse_u32("--min_depth <MIN_DEPTH>", need(tok, i, "--min_depth"));
+    else if (a == "--careful") prm.careful = 1;
+    else return false;
+    return true;
+}
+
+static bool filter_option(const std::vector<Token>& tok, size_t& i, FilterArgs& f) {
+    const std::string& a = tok[i].text;
+    if (a == "--in1") f.in1 = need(tok, i, "--in1 <IN1>");
+    else if (a == "--in2") f.in2 = need(tok, i, "--in2 <IN2>");
+    else if (a == "--out1") f.out1 = need(tok, i, "--out1 <OUT1>");
+    else if (a == "--out2") f.out2 = need(tok, i, "--out2 <OUT2>");
+    else if (a == "--orientation") f.orientation = need(tok, i, "--orientation <ORIENTATION>");
+    else if (a == "--low") f.low = parse_f64("--low <LOW>", need(tok, i, "--low"));
+    else if (a == "--high") f.high = parse_f64("--high <HIGH>", need(tok, i, "--high"));
+    else return false;
+    return true;
+}
+
+static bool common_option(const std::vector<Token>& tok, size_t& i, CommonArgs& c) {
+    const std::string& a = tok[i].text;
+    if (a == "--device") c.device = (int)parse_u32("--device", need(tok, i, "--device"));
+    else if (a == "--quiet") c.quiet = true;
+    else if (a == "--host-parse") c.host_parse = true;
+    else return false;
+    return true;
+}
+
+// A token that is no option of the command: an error when it looks like an option, else a positional argument.
+static void positional(const std::string& a, std::vector<std::string>& pos) {
+    if (a.size() > 1 && a[0] == '-' && a != "-") usage_error("unexpected argument '" + a + "' found");
+    pos.push_back(a);
+}
+
+// Contexts on `gpus` GPUs from c.device on; the process exits when there is no usable one.
+static std::vector<pp_ctx*> create_contexts(const CommonArgs& c, int gpus) {
+    const int base = restrict_visible_devices(c.device, gpus) ? 0 : c.device;
+    std::vector<pp_ctx*> ctxs(gpus, nullptr);
+    for (int g = 0; g < gpus; ++g)
+        if (pp_create(base + g, &ctxs[g]) != PP_OK) quit_with_error("no usable Blackwell (sm_100) GPU: this build has no CPU fallback");
+    if (c.host_parse) pp_set_parser(ctxs[0], 1);
+    return ctxs;
+}
+
+static void check(int rc, const std::vector<pp_ctx*>& ctxs) {
+    if (rc == PP_OK) return;
+    std::string m = pp_last_error(ctxs[0]);
+    for (auto c : ctxs) pp_destroy(c);
+    quit_with_error(m);
+}
+
 int main(int argc, char** argv) {
     mark("main");
     if (argc < 2) { help(); return 2; }
     std::string cmd = argv[1];
     if (cmd == "-h" || cmd == "--help") { help(); return 0; }
     if (cmd == "-V" || cmd == "--version") { puts("Polypolish v0.6.1"); return 0; }
-    int device = 0, gpus = 1;
-    bool quiet = false, host_parse = false;
-    std::vector<Token> tok;
-    auto need = [&](size_t& i, const char* flag) -> const char* {
-        if (i + 1 >= tok.size()) usage_error(std::string("a value is required for '") + flag + "' but none was supplied");
-        return tok[++i].text.c_str();
-    };
+    CommonArgs common;
     if (cmd == "polish") {
         pp_polish_params prm{0.2, 0.5, 10, 5, 0};
         std::string debug;
+        int gpus = 1;
         std::vector<std::string> pos;
-        tok = normalise_args(argc, argv, 2, "ivmd");
+        const std::vector<Token> tok = normalise_args(argc, argv, 2, "ivmd");
         for (size_t i = 0; i < tok.size(); ++i) {
             const std::string& a = tok[i].text;
             if (tok[i].positional) { pos.push_back(a); continue; }
             if (a == "-h" || a == "--help") { help_polish(); return 0; }
             else if (a == "-V" || a == "--version") { puts("Polypolish-polish v0.6.1"); return 0; }
-            else if (a == "--debug") debug = need(i, "--debug <DEBUG>");
-            else if (a == "-i" || a == "--fraction_invalid") prm.fraction_invalid = parse_f64("--fraction_invalid <FRACTION_INVALID>", need(i, "--fraction_invalid"));
-            else if (a == "-v" || a == "--fraction_valid") prm.fraction_valid = parse_f64("--fraction_valid <FRACTION_VALID>", need(i, "--fraction_valid"));
-            else if (a == "-m" || a == "--max_errors") prm.max_errors = parse_u32("--max_errors <MAX_ERRORS>", need(i, "--max_errors"));
-            else if (a == "-d" || a == "--min_depth") prm.min_depth = parse_u32("--min_depth <MIN_DEPTH>", need(i, "--min_depth"));
-            else if (a == "--careful") prm.careful = 1;
-            else if (a == "--device") device = (int)parse_u32("--device", need(i, "--device"));
-            else if (a == "--gpus") gpus = (int)parse_u32("--gpus", need(i, "--gpus"));
-            else if (a == "--quiet") quiet = true;
-            else if (a == "--host-parse") host_parse = true;
-            else if (a.size() > 1 && a[0] == '-' && a != "-") usage_error("unexpected argument '" + a + "' found");
-            else pos.push_back(a);
+            else if (a == "--debug") debug = need(tok, i, "--debug <DEBUG>");
+            else if (a == "--gpus") gpus = (int)parse_u32("--gpus", need(tok, i, "--gpus"));
+            else if (!polish_option(tok, i, prm) && !common_option(tok, i, common)) positional(a, pos);
         }
         if (pos.empty()) usage_error("the following required arguments were not provided:\n  <ASSEMBLY>");
         if (gpus < 1) gpus = 1;
-        const int base = restrict_visible_devices(device, gpus) ? 0 : device;
-        std::vector<pp_ctx*> ctxs(gpus, nullptr);
-        for (int g = 0; g < gpus; ++g)
-            if (pp_create(base + g, &ctxs[g]) != PP_OK) quit_with_error("no usable Blackwell (sm_100) GPU: this build has no CPU fallback");
+        const std::vector<pp_ctx*> ctxs = create_contexts(common, gpus);
         mark("contexts created");
-        if (host_parse) pp_set_parser(ctxs[0], 1);
         std::vector<const char*> sams;
         for (size_t i = 1; i < pos.size(); ++i) sams.push_back(pos[i].c_str());
         char* out = nullptr;
         uint64_t n = 0;
-        if (!quiet) fprintf(stderr, "Starting Polypolish polish (B200 build %s, %d GPU%s)\n\n", pp_version(), gpus, gpus > 1 ? "s" : "");
-        int rc = pp_polish_files_multi(ctxs.data(), gpus, pos[0].c_str(), sams.data(), (int)sams.size(), &prm, debug.empty() ? nullptr : debug.c_str(), &out, &n, quiet ? 0 : 1);
-        if (rc != PP_OK) { std::string m = pp_last_error(ctxs[0]); for (auto c : ctxs) pp_destroy(c); quit_with_error(m); }
+        if (!common.quiet) fprintf(stderr, "Starting Polypolish polish (B200 build %s, %d GPU%s)\n\n", pp_version(), gpus, gpus > 1 ? "s" : "");
+        check(pp_polish_files_multi(ctxs.data(), gpus, pos[0].c_str(), sams.data(), (int)sams.size(), &prm, debug.empty() ? nullptr : debug.c_str(),
+                                    &out, &n, common.quiet ? 0 : 1), ctxs);
         mark("polished");
         fwrite(out, 1, n, stdout);
-        if (!quiet) fprintf(stderr, "Finished!\n");
+        if (!common.quiet) fprintf(stderr, "Finished!\n");
         mark("output written");
         // A one-shot process has nothing left to do: the contexts, the driver's tear-down and the runtime's static destructors
         // (30 - 1000 ms on these boxes) are skipped - the kernel reclaims everything.  Output files first.
@@ -213,46 +262,31 @@ int main(int argc, char** argv) {
         _exit(0);
     }
     if (cmd == "filter") {
-        std::string in1, in2, out1, out2, orientation = "auto";
-        double low = 0.1, high = 99.9;
-        tok = normalise_args(argc, argv, 2, "");
+        FilterArgs f;
+        const std::vector<Token> tok = normalise_args(argc, argv, 2, "");
         for (size_t i = 0; i < tok.size(); ++i) {
             const std::string& a = tok[i].text;
             if (tok[i].positional) usage_error("unexpected argument '" + a + "' found");
             if (a == "-h" || a == "--help") { help_filter(); return 0; }
             else if (a == "-V" || a == "--version") { puts("Polypolish-filter v0.6.1"); return 0; }
-            else if (a == "--in1") in1 = need(i, "--in1 <IN1>");
-            else if (a == "--in2") in2 = need(i, "--in2 <IN2>");
-            else if (a == "--out1") out1 = need(i, "--out1 <OUT1>");
-            else if (a == "--out2") out2 = need(i, "--out2 <OUT2>");
-            else if (a == "--orientation") orientation = need(i, "--orientation <ORIENTATION>");
-            else if (a == "--low") low = parse_f64("--low <LOW>", need(i, "--low"));
-            else if (a == "--high") high = parse_f64("--high <HIGH>", need(i, "--high"));
-            else if (a == "--device") device = (int)parse_u32("--device", need(i, "--device"));
-            else if (a == "--quiet") quiet = true;
-            else if (a == "--host-parse") host_parse = true;
-            else usage_error("unexpected argument '" + a + "' found");
+            else if (!filter_option(tok, i, f) && !common_option(tok, i, common)) usage_error("unexpected argument '" + a + "' found");
         }
-        if (in1.empty() || in2.empty() || out1.empty() || out2.empty())
+        if (f.in1.empty() || f.in2.empty() || f.out1.empty() || f.out2.empty())
             usage_error("the following required arguments were not provided:\n  --in1 <IN1>\n  --in2 <IN2>\n  --out1 <OUT1>\n  --out2 <OUT2>");
-        const int base = restrict_visible_devices(device, 1) ? 0 : device;
-        pp_ctx* ctx = nullptr;
-        if (pp_create(base, &ctx) != PP_OK) quit_with_error("no usable Blackwell (sm_100) GPU: this build has no CPU fallback");
-        if (host_parse) pp_set_parser(ctx, 1);
-        if (!quiet) fprintf(stderr, "Starting Polypolish filter (B200 build %s)\n\n", pp_version());
-        int rc = pp_filter_files(ctx, in1.c_str(), in2.c_str(), out1.c_str(), out2.c_str(), orientation.c_str(), low, high, quiet ? 0 : 1);
-        if (rc != PP_OK) { std::string m = pp_last_error(ctx); pp_destroy(ctx); quit_with_error(m); }
-        if (!quiet) fprintf(stderr, "Finished!\n");
+        const std::vector<pp_ctx*> ctxs = create_contexts(common, 1);
+        if (!common.quiet) fprintf(stderr, "Starting Polypolish filter (B200 build %s)\n\n", pp_version());
+        check(pp_filter_files(ctxs[0], f.in1.c_str(), f.in2.c_str(), f.out1.c_str(), f.out2.c_str(), f.orientation.c_str(), f.low, f.high,
+                              common.quiet ? 0 : 1), ctxs);
+        if (!common.quiet) fprintf(stderr, "Finished!\n");
         fflush(stderr);
         _exit(0);                                           // (see `polish`: nothing left to do, the tear-down is skipped)
     }
     if (cmd == "filter-polish") {
         // ADDITIVE (not in the reference): `filter` and `polish` of its output as one command, no intermediate files unless named
         pp_polish_params prm{0.2, 0.5, 10, 5, 0};
-        std::string in1, in2, out1, out2, orientation = "auto";
-        double low = 0.1, high = 99.9;
+        FilterArgs f;
         std::vector<std::string> pos;
-        tok = normalise_args(argc, argv, 2, "ivmd");
+        const std::vector<Token> tok = normalise_args(argc, argv, 2, "ivmd");
         for (size_t i = 0; i < tok.size(); ++i) {
             const std::string& a = tok[i].text;
             if (tok[i].positional) { pos.push_back(a); continue; }
@@ -262,38 +296,19 @@ int main(int argc, char** argv) {
                 puts("Options: those of `filter` (--out1 / --out2 optional: written only when given) and of `polish` (except --debug)");
                 return 0;
             }
-            else if (a == "--in1") in1 = need(i, "--in1 <IN1>");
-            else if (a == "--in2") in2 = need(i, "--in2 <IN2>");
-            else if (a == "--out1") out1 = need(i, "--out1 <OUT1>");
-            else if (a == "--out2") out2 = need(i, "--out2 <OUT2>");
-            else if (a == "--orientation") orientation = need(i, "--orientation <ORIENTATION>");
-            else if (a == "--low") low = parse_f64("--low <LOW>", need(i, "--low"));
-            else if (a == "--high") high = parse_f64("--high <HIGH>", need(i, "--high"));
-            else if (a == "-i" || a == "--fraction_invalid") prm.fraction_invalid = parse_f64("--fraction_invalid <FRACTION_INVALID>", need(i, "--fraction_invalid"));
-            else if (a == "-v" || a == "--fraction_valid") prm.fraction_valid = parse_f64("--fraction_valid <FRACTION_VALID>", need(i, "--fraction_valid"));
-            else if (a == "-m" || a == "--max_errors") prm.max_errors = parse_u32("--max_errors <MAX_ERRORS>", need(i, "--max_errors"));
-            else if (a == "-d" || a == "--min_depth") prm.min_depth = parse_u32("--min_depth <MIN_DEPTH>", need(i, "--min_depth"));
-            else if (a == "--careful") prm.careful = 1;
-            else if (a == "--device") device = (int)parse_u32("--device", need(i, "--device"));
-            else if (a == "--quiet") quiet = true;
-            else if (a == "--host-parse") host_parse = true;
-            else if (a.size() > 1 && a[0] == '-' && a != "-") usage_error("unexpected argument '" + a + "' found");
-            else pos.push_back(a);
+            else if (!filter_option(tok, i, f) && !polish_option(tok, i, prm) && !common_option(tok, i, common)) positional(a, pos);
         }
-        if (in1.empty() || in2.empty() || pos.size() != 1)
+        if (f.in1.empty() || f.in2.empty() || pos.size() != 1)
             usage_error("the following required arguments were not provided:\n  --in1 <IN1>\n  --in2 <IN2>\n  <ASSEMBLY>");
-        const int base = restrict_visible_devices(device, 1) ? 0 : device;
-        pp_ctx* ctx = nullptr;
-        if (pp_create(base, &ctx) != PP_OK) quit_with_error("no usable Blackwell (sm_100) GPU: this build has no CPU fallback");
-        if (host_parse) pp_set_parser(ctx, 1);
-        if (!quiet) fprintf(stderr, "Starting Polypolish filter + polish (B200 build %s)\n\n", pp_version());
+        const std::vector<pp_ctx*> ctxs = create_contexts(common, 1);
+        if (!common.quiet) fprintf(stderr, "Starting Polypolish filter + polish (B200 build %s)\n\n", pp_version());
         char* out = nullptr;
         uint64_t n = 0;
-        int rc = pp_filter_polish_files(ctx, pos[0].c_str(), in1.c_str(), in2.c_str(), out1.empty() ? nullptr : out1.c_str(), out2.empty() ? nullptr : out2.c_str(),
-                                        orientation.c_str(), low, high, &prm, &out, &n, quiet ? 0 : 1);
-        if (rc != PP_OK) { std::string m = pp_last_error(ctx); pp_destroy(ctx); quit_with_error(m); }
+        check(pp_filter_polish_files(ctxs[0], pos[0].c_str(), f.in1.c_str(), f.in2.c_str(), f.out1.empty() ? nullptr : f.out1.c_str(),
+                                     f.out2.empty() ? nullptr : f.out2.c_str(), f.orientation.c_str(), f.low, f.high, &prm, &out, &n,
+                                     common.quiet ? 0 : 1), ctxs);
         fwrite(out, 1, n, stdout);
-        if (!quiet) fprintf(stderr, "Finished!\n");
+        if (!common.quiet) fprintf(stderr, "Finished!\n");
         if (fflush(stdout) != 0 || ferror(stdout)) quit_with_error("unable to write to stdout");
         fflush(stderr);
         _exit(0);

@@ -105,42 +105,43 @@ bool write_filtered(const MateFile& m, const uint8_t* pass, const std::string& o
     return (fclose(f) == 0) && ok;
 }
 
-std::string thousands(uint64_t v) {
-    std::string s = std::to_string(v), o;
-    int n = (int)s.size();
-    for (int i = 0; i < n; ++i) { o += s[i]; if ((n - 1 - i) % 3 == 0 && i != n - 1) o += ','; }
-    return o;
-}
-
 }  // namespace
+
+int pp::check_filter_args(pp_ctx* ctx, const char* in1, const char* in2, const char* out1, const char* out2, const char* orientation,
+                          double low, double high, pp_filter_params* prm) {
+    {   // check_inputs filter.rs:40-53
+        std::vector<std::string> a = {in1, in2};
+        if (out1) a.push_back(out1);
+        if (out2) a.push_back(out2);
+        for (size_t i = 0; i < a.size(); ++i)
+            for (size_t j = 0; j < i; ++j)
+                if (a[i] == a[j]) return pp_ctx_fail(ctx, PP_ERR_INPUT, "--in1, --in2, --out1 and --out2 must all have unique values");
+    }
+    if (!(low > 0.0 && low < 50.0)) return pp_ctx_fail(ctx, PP_ERR_INPUT, "--low must be greater than 0 and less than 50");
+    if (!(high > 50.0 && high < 100.0)) return pp_ctx_fail(ctx, PP_ERR_INPUT, "--high must be greater than 50 and less than 100");
+    const std::string o = orientation;
+    prm->orientation = o == "auto" ? -1 : o == "fr" ? 0 : o == "rf" ? 1 : o == "ff" ? 2 : o == "rr" ? 3 : 4;
+    prm->low_pct = low;
+    prm->high_pct = high;
+    prm->n_names = 0;
+    return PP_OK;
+}
 
 extern "C" int pp_filter_files(pp_ctx* ctx, const char* in1, const char* in2, const char* out1, const char* out2,
                                const char* orientation, double low, double high, int verbose) {
     if (!ctx) return PP_ERR_ARG;
     if (!in1 || !in2 || !out1 || !out2 || !orientation) return pp_ctx_fail(ctx, PP_ERR_ARG, "pp_filter_files: null argument");
-    // check_inputs filter.rs:40-53
-    {
-        std::string a[4] = {in1, in2, out1, out2};
-        for (int i = 0; i < 4; ++i)
-            for (int j = 0; j < i; ++j)
-                if (a[i] == a[j]) return pp_ctx_fail(ctx, PP_ERR_INPUT, "--in1, --in2, --out1 and --out2 must all have unique values");
-    }
-    if (!(low > 0.0 && low < 50.0)) return pp_ctx_fail(ctx, PP_ERR_INPUT, "--low must be greater than 0 and less than 50");
-    if (!(high > 50.0 && high < 100.0)) return pp_ctx_fail(ctx, PP_ERR_INPUT, "--high must be greater than 50 and less than 100");
-
     pp_filter_params prm;
-    std::string o = orientation;
-    prm.orientation = o == "auto" ? -1 : o == "fr" ? 0 : o == "rf" ? 1 : o == "ff" ? 2 : o == "rr" ? 3 : 4;
-    prm.low_pct = low;
-    prm.high_pct = high;
-    prm.n_names = 0;
+    const int arc = pp::check_filter_args(ctx, in1, in2, out1, out2, orientation, low, high, &prm);
+    if (arc != PP_OK) return arc;
+
     pp_filter_result res;
     memset(&res, 0, sizeof res);
     const char* ins[2] = {in1, in2};
     const char* outs[2] = {out1, out2};
     const char* nm[4] = {"fr", "rf", "ff", "rr"};
     auto log_thresholds = [&]() {
-        for (int i = 0; i < 4; ++i) fprintf(stderr, "%s: %s pairs\n", nm[i], thousands(res.pairs[i]).c_str());
+        for (int i = 0; i < 4; ++i) fprintf(stderr, "%s: %s pairs\n", nm[i], pp::thousands(res.pairs[i]).c_str());
         fprintf(stderr, "\n%s correct orientation: %s\n\n", prm.orientation < 0 ? "Automatically determined" : "User-specified",
                 res.orientation < 4 ? nm[res.orientation] : orientation);
         fprintf(stderr, "Low threshold:  %u\nHigh threshold: %u\n\n", res.low, res.high);
@@ -153,12 +154,12 @@ extern "C" int pp_filter_files(pp_ctx* ctx, const char* in1, const char* in2, co
         int rc = pp_filter_files_device(ctx, in1, in2, out1, out2, &prm, &res, &fs, nullptr);
         if (rc == PP_OK) {
             if (verbose) {
-                for (int k = 0; k < 2; ++k) fprintf(stderr, "%s: %s alignments\n", ins[k], thousands(fs.alignments[k]).c_str());
+                for (int k = 0; k < 2; ++k) fprintf(stderr, "%s: %s alignments\n", ins[k], pp::thousands(fs.alignments[k]).c_str());
                 log_thresholds();
                 for (int k = 0; k < 2; ++k)
-                    fprintf(stderr, "Filtering %s:\n  %s pass\n  %s fail\n\n", ins[k], thousands(fs.pass[k]).c_str(), thousands(fs.fail[k]).c_str());
-                fprintf(stderr, "Alignments before filtering: %s\nAlignments after filtering:  %s\n\n", thousands(fs.alignments[0] + fs.alignments[1]).c_str(),
-                        thousands(fs.pass[0] + fs.pass[1]).c_str());
+                    fprintf(stderr, "Filtering %s:\n  %s pass\n  %s fail\n\n", ins[k], pp::thousands(fs.pass[k]).c_str(), pp::thousands(fs.fail[k]).c_str());
+                fprintf(stderr, "Alignments before filtering: %s\nAlignments after filtering:  %s\n\n", pp::thousands(fs.alignments[0] + fs.alignments[1]).c_str(),
+                        pp::thousands(fs.pass[0] + fs.pass[1]).c_str());
                 fprintf(stderr, "device text path: %.3f ms (SAM to HBM %.3f ms, filtered SAM to files %.3f ms), %u kernels; filter kernels %.3f ms\n", fs.total_ms,
                         fs.h2d_ms, fs.d2h_ms, fs.launches, res.timing.total_ms);
                 fprintf(stderr, "  phases (wall ms): upload+index+parse %.1f, intern+verify+emit %.1f, filter %.1f, output offsets %.1f, output bytes %.1f, download+write %.1f\n",
@@ -177,7 +178,7 @@ extern "C" int pp_filter_files(pp_ctx* ctx, const char* in1, const char* in2, co
     std::string err;
     for (int k = 0; k < 2; ++k) {
         if (!load_mate(m[k], names, err)) return pp_ctx_fail(ctx, PP_ERR_INPUT, err.c_str());
-        if (verbose) fprintf(stderr, "%s: %s alignments\n", m[k].path.c_str(), thousands(m[k].name_id.size()).c_str());
+        if (verbose) fprintf(stderr, "%s: %s alignments\n", m[k].path.c_str(), pp::thousands(m[k].name_id.size()).c_str());
         if (m[0].name_id.empty() && (k == 0 || m[1].name_id.empty()))      // alignments.is_empty() filter.rs:141-143
             return pp_ctx_fail(ctx, PP_ERR_INPUT, ("no alignments found in \"" + m[k].path + "\"").c_str());
     }
@@ -202,10 +203,10 @@ extern "C" int pp_filter_files(pp_ctx* ctx, const char* in1, const char* in2, co
         if (!write_filtered(m[k], passes[k], outs[k], np, nf))
             return pp_ctx_fail(ctx, PP_ERR_IO, ("unable to write alignments to \"" + std::string(outs[k]) + "\"").c_str());
         after += np;
-        if (verbose) fprintf(stderr, "Filtering %s:\n  %s pass\n  %s fail\n\n", m[k].path.c_str(), thousands(np).c_str(), thousands(nf).c_str());
+        if (verbose) fprintf(stderr, "Filtering %s:\n  %s pass\n  %s fail\n\n", m[k].path.c_str(), pp::thousands(np).c_str(), pp::thousands(nf).c_str());
     }
     if (verbose) {
-        fprintf(stderr, "Alignments before filtering: %s\nAlignments after filtering:  %s\n\n", thousands(before).c_str(), thousands(after).c_str());
+        fprintf(stderr, "Alignments before filtering: %s\nAlignments after filtering:  %s\n\n", pp::thousands(before).c_str(), pp::thousands(after).c_str());
         fprintf(stderr, "device path: %.3f ms, %u kernels\n", res.timing.total_ms, res.timing.launches);
     }
     return PP_OK;

@@ -48,10 +48,13 @@ struct AlignedBytes {
     void clear() { n = 0; }
 };
 
-struct Error {
-    int code;
-    std::string msg;
-};
+// 1234567 -> "1,234,567" (num_format Locale::en, what the reference's logs print)
+std::string thousands(uint64_t v);
+
+// The argument checks of `polypolish filter` (check_inputs filter.rs:40-53, the --low / --high ranges) and its parameters, the
+// orientation text as a code.  out1 / out2 may be null (not written).  PP_OK, or the error, reported on ctx.
+int check_filter_args(pp_ctx* ctx, const char* in1, const char* in2, const char* out1, const char* out2, const char* orientation,
+                      double low, double high, pp_filter_params* prm);
 
 }  // namespace pp
 
