@@ -241,6 +241,11 @@ typedef struct pp_pack pp_pack;
  * QNAME grouping, source sequence of SEQ="*" records. */
 pp_pack* pp_pack_create(const pp_fasta* f, int careful);
 void pp_pack_free(pp_pack* p);
+/* A BAM file (recognised by content: a BGZF block that inflates to "BAM\1", never by its name; pipes are always SAM) is parsed as
+ * its SAM text: the stored header text, then one line per record (SAMv1 §4.2's columns with the NM and ZP tags, a CG:B:I array in
+ * place of the long-CIGAR placeholder), so results, messages and "(line N)" numbers are those of that text.  PP_ERR_IO, with a
+ * message naming the file, for what only BAM can get wrong: not BGZF, a CRC32 / ISIZE mismatch, a record past its block_size or
+ * past the end of the data, a refID / next_refID out of range, malformed optional fields, no BGZF end-of-file block. */
 int pp_pack_add_sam_file(pp_pack* p, const char* path);                        /* PP_OK / PP_ERR_INPUT / PP_ERR_IO */
 /* big files are parsed by several host threads (same result, same errors); 0 threads = one per hardware thread */
 int pp_pack_set_threads(pp_pack* p, uint32_t n_threads, uint64_t min_chunk_bytes);
@@ -282,8 +287,11 @@ typedef struct {
 } pp_tok_stats;
 int pp_tok_begin(pp_ctx* ctx, const pp_fasta* assembly, int careful, int seq_bits /* 4 | 8 */);
 int pp_tok_add_text(pp_ctx* ctx, const char* text, size_t len, pp_tok_stats* stats /* may be NULL */);
+/* A BAM file (as in pp_pack_add_sam_file) is inflated on the host, its image crosses PCIe and is decoded one record per thread;
+ * the result is the same as for its SAM text.  Its stats count records as lines, and h2d_ms covers read, inflate, record walk
+ * and PCIe.  Anything the host must word (a structural fault included) is PP_TOK_HOST.  pp_tok_prefetch of a BAM does nothing. */
 int pp_tok_add_file(pp_ctx* ctx, const char* path, pp_tok_stats* stats /* may be NULL */);
-/* Several files in order, pipelined: file i+1 streams into a second text buffer while file i is tokenised. */
+/* Several files in order, pipelined: file i+1 streams into a second text buffer while file i is tokenised.  SAM and BAM may mix. */
 int pp_tok_add_files(pp_ctx* ctx, const char* const* paths, int n_paths, pp_tok_stats* stats /* [n_paths] or NULL */);
 /* Optional, any time after pp_create: start streaming `path` into HBM in the background (one outstanding upload);
  * the next pp_tok_add_file(s) that starts with the same path picks it up.  Lets the upload overlap the FASTA load. */
@@ -301,7 +309,7 @@ int pp_tok_set_shard(pp_ctx* ctx, const uint32_t* local_of, uint32_t n_contigs_t
 /* n byte ranges of a SAM file for n GPUs: cuts[0] = 0, cuts[n] = the file size, every other cut is the start of a line whose QNAME
  * differs from the line before it, so that no read group (alignment.rs:214-272) is split.  PP_ERR_IO: not a plain file / a line longer
  * than 1 MiB.  (pp_polish_files_multi gives range g of every file to GPU g, then the GPUs exchange read groups by contig.) */
-int pp_sam_split_ranges(const char* path, int n, uint64_t* cuts /* [n + 1] */);
+int pp_sam_split_ranges(const char* path, int n, uint64_t* cuts /* [n + 1] */);   /* SAM only: PP_ERR_IO for a BAM file */
 /* Multi-GPU ingestion, the building blocks of pp_polish_files_multi (polish.rs:109-134 load_alignments over N GPUs).  Per context g:
  *   pp_tok_begin -> pp_tok_set_ranges(off, len, n_files): this context reads only bytes [off[f], off[f] + len[f]) of file f
  *   (range g of pp_sam_split_ranges) -> pp_tok_add_files(the same n_files paths on every context).
@@ -310,6 +318,7 @@ int pp_sam_split_ranges(const char* path, int n, uint64_t* cuts /* [n + 1] */);
  * shard_contigs[g] or 0xFFFFFFFF; peer copies on the device, global SAM order = (file, range, line)), marks the foreign records
  * PP_FLAG_GHOST, installs shard_contigs[g] as context g's draft and bins: every context is then ready for pp_polish_resident.
  * PP_TOK_HOST: more than 32 contexts / 64 files, or something the host path must look at.  n_aln_total = aligned records read. */
+/* (SAM only: pp_tok_add_files answers PP_TOK_HOST when a file of a ranged list is BAM; pp_polish_files_multi cuts BAM files by record.) */
 int pp_tok_set_ranges(pp_ctx* ctx, const uint64_t* off, const uint64_t* len, int n_files);
 int pp_tok_exchange_finish(pp_ctx* const* ctxs, int n_ctx, const uint32_t* owner, uint32_t n_contigs_total, const uint32_t* const* local_of,
                            const pp_contigs* shard_contigs /* [n_ctx] */, uint64_t* n_aln_total);
@@ -346,12 +355,14 @@ void pp_shards_free(pp_shards* s);
  * reference's polish::polish (polish.rs:26-38) and filter::filter (filter.rs:26-37)).
  * out_fasta receives exactly what the reference prints to stdout; free with pp_free.
  * pp_polish_files parses its SAM files with the device tokeniser (pp_tok_*) unless pp_set_parser(ctx, 1), a --debug run, or
- * PP_TOK_HOST / a data error send it through pp_pack_*. */
+ * PP_TOK_HOST / a data error send it through pp_pack_*.  Any of `sams` may be a BAM file instead (pp_pack_add_sam_file): same output,
+ * log and errors as its SAM text. */
 int pp_polish_files(pp_ctx* ctx, const char* assembly, const char* const* sams, int n_sams,
                     const pp_polish_params* params, const char* debug_path, char** out_fasta,
                     uint64_t* out_len, int verbose /* 1: reference-style log on stderr */);
 /* the same command over several GPUs of one box: contigs shard across ctxs[0..n_ctx) (one host thread per GPU); every GPU tokenises
- * its byte range of every SAM file and the read groups change GPUs on the device (pp_tok_set_ranges / pp_tok_exchange_finish) */
+ * its byte range of every SAM file and the read groups change GPUs on the device (pp_tok_set_ranges / pp_tok_exchange_finish).  A BAM
+ * file is inflated once on the host and every GPU decodes its range of the records, cut between read groups. */
 int pp_polish_files_multi(pp_ctx* const* ctxs, int n_ctx, const char* assembly, const char* const* sams, int n_sams,
                           const pp_polish_params* params, const char* debug_path, char** out_fasta,
                           uint64_t* out_len, int verbose);
@@ -404,6 +415,8 @@ uint64_t pp_synth_total_bp(const pp_synth* s);    /* draft bases */
 uint64_t pp_synth_n_pairs(const pp_synth* s);
 int pp_synth_write_fasta(const pp_synth* s, const char* path, int truth /* 0 = draft */);
 int pp_synth_write_sam(const pp_synth* s, int mate /* 1 | 2 */, const char* path);
+/* the same records as BAM (BGZF, level 6, with the end-of-file block), compressed on the worker threads of pp_synth_set_threads */
+int pp_synth_write_bam(const pp_synth* s, int mate /* 1 | 2 */, const char* path);
 pp_fasta* pp_synth_fasta(const pp_synth* s);      /* the draft as a loaded assembly (free with pp_fasta_free) */
 int pp_synth_feed_pack(const pp_synth* s, int mate, pp_pack* pack); /* same text, streamed into the packer */
 

@@ -565,12 +565,14 @@ class Synth:
         L.pp_synth_set_threads.argtypes = [C.c_void_p, C.c_uint32]
         L.pp_synth_set_threads(self.h, int(n_threads))
 
-    def write(self, directory):
-        """draft FASTA + one SAM per mate; returns (fasta, [sam1, sam2])."""
+    def write(self, directory, bam=False):
+        """draft FASTA + one SAM (bam=True: BAM, the same records) per mate; returns (fasta, [file1, file2])."""
         d = str(directory)
-        fa, s1, s2 = os.path.join(d, "draft.fasta"), os.path.join(d, "reads_1.sam"), os.path.join(d, "reads_2.sam")
-        for rc in (lib().pp_synth_write_fasta(self.h, fa.encode(), 0), lib().pp_synth_write_sam(self.h, 1, s1.encode()),
-                   lib().pp_synth_write_sam(self.h, 2, s2.encode())):
+        L = lib()
+        L.pp_synth_write_bam.argtypes = [C.c_void_p, C.c_int, C.c_char_p]
+        ext, wr = (".bam", L.pp_synth_write_bam) if bam else (".sam", L.pp_synth_write_sam)
+        fa, s1, s2 = os.path.join(d, "draft.fasta"), os.path.join(d, "reads_1" + ext), os.path.join(d, "reads_2" + ext)
+        for rc in (L.pp_synth_write_fasta(self.h, fa.encode(), 0), wr(self.h, 1, s1.encode()), wr(self.h, 2, s2.encode())):
             if rc != PP_OK:
                 raise PolypolishError(rc, "synthetic data could not be written")
         return fa, [s1, s2]

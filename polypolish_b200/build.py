@@ -18,7 +18,7 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-Wall,-Wno-unus
           "-fmad=false"]   # IEEE double semantics: no FMA contraction anywhere near the vote
 
 LIB_SOURCES = ["polish_kernels.cu", "filter_kernels.cu", "tok_kernels.cu", "fasta.cpp", "sam_pack.cpp", "filter_pack.cpp",
-               "host_api.cpp", "synth.cpp", "shard.cpp"]
+               "host_api.cpp", "synth.cpp", "shard.cpp", "bam.cpp"]
 CLI_SOURCES = ["cli_main.cpp"]
 
 
@@ -27,7 +27,7 @@ def _stale(target, sources):
         return True
     t = os.path.getmtime(target)
     deps = list(sources) + [os.path.join(CSRC, "pp_internal.h"), os.path.join(CSRC, "nib_utils.h"), os.path.join(CSRC, "pp_ctx.cuh"), os.path.join(CSRC, "polish_dev.cuh"),
-                            os.path.join(CSRC, "tok_line.h"), os.path.join(CSRC, "tok_table.h"), os.path.join(CSRC, "filter_dev.h"), os.path.join(CSRC, "tok_strip.h"), os.path.join(ROOT, "include", "pp_abi.h"),
+                            os.path.join(CSRC, "tok_line.h"), os.path.join(CSRC, "tok_table.h"), os.path.join(CSRC, "filter_dev.h"), os.path.join(CSRC, "tok_strip.h"), os.path.join(CSRC, "bam_rec.h"), os.path.join(ROOT, "include", "pp_abi.h"),
                             os.path.abspath(__file__)]
     return any(os.path.getmtime(d) > t for d in deps if os.path.exists(d))
 

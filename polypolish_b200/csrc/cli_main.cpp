@@ -85,6 +85,7 @@ static void help_polish() {               // main.rs:77-108
     puts("  -V, --version");
     puts("          Print version");
     puts("\nB200 build, additive options: --device <N> (first GPU, default 0), --gpus <N> (contigs shard over N GPUs), --quiet, --host-parse");
+    puts("Alignment files may also be BAM (recognised by content, not by name)");
 }
 
 // clap accepts `--name=value`, `-m5` / `-m=5` and a `--` separator (everything after it is positional): normalise those forms

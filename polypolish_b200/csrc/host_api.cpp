@@ -274,6 +274,7 @@ static bool split_ranges(const char* path, int n, std::vector<uint64_t>& cut) {
 
 extern "C" int pp_sam_split_ranges(const char* path, int n, uint64_t* cuts) {
     if (!path || n < 1 || !cuts) return PP_ERR_ARG;
+    if (pp::is_bam(path)) return PP_ERR_IO;                          // byte ranges of a BAM are not record boundaries
     std::vector<uint64_t> c;
     if (!split_ranges(path, n, c)) return PP_ERR_IO;
     std::copy(c.begin(), c.end(), cuts);
@@ -343,7 +344,8 @@ static int load_fused(pp_ctx* ctx, const pp_fasta* fa, const pp_contigs& contigs
 // Several GPUs, no host in the middle: the host only decides which contig goes where (longest contig first onto the lightest shard)
 // and where to cut the files; the text, the records and the shards never pass through host memory as arrays.  Every GPU reads ITS
 // byte range of every file (cut between read groups), tokenises it, and the read groups are exchanged between the GPUs
-// (tok_kernels.cu pp_tok_exchange_finish): 1/N of the text per PCIe link.
+// (tok_kernels.cu pp_tok_exchange_finish): 1/N of the text per PCIe link.  A BAM file is inflated once, here, and every GPU decodes
+// its range of the records of that one image (cut between read groups as well).
 static int load_device_ranges(pp_ctx* const* ctxs, uint32_t n_shards, const pp_fasta* fa, const pp_contigs& contigs,
                               const char* const* sams, int n_sams, int careful, Loaded& d) {
     std::vector<uint32_t> order(contigs.n_contigs), owner(contigs.n_contigs);
@@ -373,8 +375,17 @@ static int load_device_ranges(pp_ctx* const* ctxs, uint32_t n_shards, const pp_f
         j.resident = true;
     }
     std::vector<std::vector<uint64_t>> cuts((size_t)n_sams);
-    for (int i = 0; i < n_sams; ++i)
-        if (!split_ranges(sams[i], (int)n_shards, cuts[(size_t)i])) return PP_TOK_HOST;
+    std::vector<std::unique_ptr<pp::BamImage>> bams((size_t)n_sams);
+    for (int i = 0; i < n_sams; ++i) {
+        if (pp::is_bam(sams[i])) {
+            bams[(size_t)i].reset(new pp::BamImage());
+            std::string err;
+            if (pp::bam_load(sams[i], fa, *bams[(size_t)i], err) != PP_OK) return PP_TOK_HOST;     // the host path words the error
+            pp::bam_split(*bams[(size_t)i], (int)n_shards, cuts[(size_t)i]);
+        } else if (!split_ranges(sams[i], (int)n_shards, cuts[(size_t)i])) {
+            return PP_TOK_HOST;
+        }
+    }
     std::vector<std::vector<pp_tok_stats>> tst(n_shards, std::vector<pp_tok_stats>((size_t)n_sams));
     int rc = with_seq_bits([&](int bits) {
         std::vector<int> trc(n_shards, PP_OK);
@@ -382,10 +393,15 @@ static int load_device_ranges(pp_ctx* const* ctxs, uint32_t n_shards, const pp_f
             pp_ctx* c = ctxs[s];
             std::vector<uint64_t> off((size_t)n_sams), len((size_t)n_sams);
             uint64_t mine = 0;
-            for (int i = 0; i < n_sams; ++i) { off[(size_t)i] = cuts[(size_t)i][s]; len[(size_t)i] = cuts[(size_t)i][s + 1] - cuts[(size_t)i][s]; mine += len[(size_t)i]; }
+            for (int i = 0; i < n_sams; ++i) {
+                if (bams[(size_t)i]) continue;                          // (a BAM's range is a range of records, set below)
+                off[(size_t)i] = cuts[(size_t)i][s]; len[(size_t)i] = cuts[(size_t)i][s + 1] - cuts[(size_t)i][s]; mine += len[(size_t)i];
+            }
             int r = pp_tok_begin(c, fa, careful ? 1 : 0, bits);
             if (r == PP_OK) r = pp_tok_expect(c, mine);
             if (r == PP_OK) r = pp_tok_set_ranges(c, off.data(), len.data(), n_sams);
+            for (int i = 0; i < n_sams && r == PP_OK; ++i)
+                if (bams[(size_t)i]) r = pp_tok_set_bam_range(c, i, bams[(size_t)i].get(), cuts[(size_t)i][s], cuts[(size_t)i][s + 1]);
             if (r == PP_OK) r = pp_tok_add_files(c, sams, n_sams, tst[s].data());
             trc[s] = r;
             if (r != PP_OK && r != PP_TOK_HOST && r != PP_TOK_NEED8) d.jobs[s].err = pp_last_error(c);
@@ -412,8 +428,13 @@ static int load_device_ranges(pp_ctx* const* ctxs, uint32_t n_shards, const pp_f
         empty_file |= na == 0;                                         // "no alignments in <file>" (alignment.rs:268-270): the host path words it
         d.log += std::string(sams[i]) + ": " + pp::thousands(na) + " alignments from " + pp::thousands(nr) + " reads\n";
         char tmp[256];
-        snprintf(tmp, sizeof tmp, "SAM tokeniser %s: %s lines in %u byte ranges, text to HBM %.3f ms, kernels %.3f ms (slowest GPU)\n", sams[i],
-                 pp::thousands(nl).c_str(), n_shards, h2d, dev);
+        if (bams[(size_t)i])
+            snprintf(tmp, sizeof tmp, "BAM decoder %s: %s records in %u ranges, read %.3f ms, inflate %.3f ms, record walk %.3f ms, image to HBM %.3f ms, "
+                     "kernels %.3f ms (slowest GPU)\n", sams[i], pp::thousands(nl).c_str(), n_shards, bams[(size_t)i]->read_ms, bams[(size_t)i]->inflate_ms,
+                     bams[(size_t)i]->walk_ms, h2d, dev);
+        else
+            snprintf(tmp, sizeof tmp, "SAM tokeniser %s: %s lines in %u byte ranges, text to HBM %.3f ms, kernels %.3f ms (slowest GPU)\n", sams[i],
+                     pp::thousands(nl).c_str(), n_shards, h2d, dev);
         d.timing += tmp;
     }
     if (empty_file) return PP_TOK_HOST;
@@ -454,9 +475,14 @@ static int load_device_one(pp_ctx* ctx, const pp_fasta* fa, const pp_contigs& co
     for (int i = 0; i < n_sams; ++i) {
         d.alns.n_aln += st[i].alignments;
         d.log += std::string(sams[i]) + ": " + pp::thousands(st[i].alignments) + " alignments from " + pp::thousands(st[i].reads) + " reads\n";
-        char tmp[256];
-        snprintf(tmp, sizeof tmp, "SAM tokeniser %s: %s lines, text to HBM %.3f ms, %u kernels %.3f ms\n", sams[i], pp::thousands(st[i].lines).c_str(),
-                 st[i].h2d_ms, st[i].launches, st[i].device_ms);
+        char tmp[320];
+        float rd = 0, inf = 0, walk = 0, up = 0;
+        if (pp_tok_bam_phases(ctx, i, &rd, &inf, &walk, &up))
+            snprintf(tmp, sizeof tmp, "BAM decoder %s: %s records, read %.3f ms, inflate %.3f ms, record walk %.3f ms, image to HBM %.3f ms, %u kernels %.3f ms\n",
+                     sams[i], pp::thousands(st[i].lines).c_str(), rd, inf, walk, up, st[i].launches, st[i].device_ms);
+        else
+            snprintf(tmp, sizeof tmp, "SAM tokeniser %s: %s lines, text to HBM %.3f ms, %u kernels %.3f ms\n", sams[i], pp::thousands(st[i].lines).c_str(),
+                     st[i].h2d_ms, st[i].launches, st[i].device_ms);
         d.timing += tmp;
     }
     d.one_job(ctx, contigs, true);

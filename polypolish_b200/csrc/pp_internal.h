@@ -1,6 +1,7 @@
 // pp_internal.h — shared host-side declarations of libpolypolish_b200 (not part of the ABI).
 #pragma once
 #include <cstdint>
+#include <cstdio>
 #include <cstring>
 #include <string>
 #include <string_view>
@@ -56,6 +57,48 @@ std::string thousands(uint64_t v);
 int check_filter_args(pp_ctx* ctx, const char* in1, const char* in2, const char* out1, const char* out2, const char* orientation,
                       double low, double high, pp_filter_params* prm);
 
+// ---- BAM input (bam.cpp) ----
+// The decoded form of a BAM file that both parsers use: the inflated stream, where each record starts, the refID -> contig table.
+struct BamImage {
+    std::string path;
+    AlignedBytes data;                  // the uncompressed stream, zero padded
+    uint64_t size = 0;                  // its bytes
+    std::vector<uint64_t> rec;          // offset of every record (its block_size field)
+    std::string header;                 // the stored header text up to its first NUL, ending in '\n' unless empty
+    uint64_t header_lines = 0;          // its lines (the SAM text's line numbers of the records start after them)
+    std::vector<std::string> ref_names; // [n_ref]
+    std::vector<uint32_t> ref_contig;   // [n_ref + 1]: contig of refID r at r + 1 (entry 0: refID -1, RNAME "*"), or PP_CONTIG_UNKNOWN
+    bool device_ok = true;              // false: a header line that is not one in SAM, a reference name with a tab / CR / LF
+    float read_ms = 0, inflate_ms = 0, walk_ms = 0;
+};
+// Content, not the name: a regular file whose first bytes are a BGZF block that inflates to "BAM\1".  Pipes are never opened.
+bool is_bam(const char* path);
+// PP_OK, or PP_ERR_IO with a message naming the file (unreadable, not BGZF, CRC32 / ISIZE mismatch, truncated, a broken record chain).
+// fa may be null (ref_contig then stays unknown).
+int bam_load(const char* path, const pp_fasta* fa, BamImage& im, std::string& err);
+// The header text and one SAM line per record (what the host packer parses).  PP_ERR_IO: a structural fault of a record.
+int bam_to_sam(const BamImage& im, std::string& out, std::string& err);
+// Record ranges of a BAM for n decoders, cut only where a read group ends (alignment.rs:255).
+void bam_split(const BamImage& im, int n, std::vector<uint64_t>& cut);
+
+// BGZF output (level `level`), compressed by `threads` threads, with the end-of-file block at close().
+class BgzfWriter {
+public:
+    BgzfWriter(const char* path, int level, unsigned threads);
+    ~BgzfWriter();
+    bool write(const void* p, size_t n);
+    bool close();
+private:
+    bool flush(bool all);
+    FILE* f_ = nullptr;
+    int level_;
+    unsigned threads_;
+    std::string buf_;
+    bool ok_ = true;
+};
+void bam_header(const std::string& text, const std::vector<std::pair<std::string, uint64_t>>& refs, std::string& out);
+bool sam_line_to_bam(std::string_view line, const std::unordered_map<std::string, int32_t>& ref_id, std::string& out);
+
 }  // namespace pp
 
 struct pp_fasta {
@@ -101,6 +144,13 @@ struct pp_pack {
 };
 
 int pp_ctx_fail(pp_ctx* ctx, int code, const char* msg);
+
+// Between pp_tok_begin and pp_tok_add_files: file `file` of the list is records [r0, r1) of an image decoded by the caller, who keeps
+// it alive until pp_tok_add_files returns (several contexts decode ranges of one image: host_api.cpp load_device_ranges).
+int pp_tok_set_bam_range(pp_ctx* ctx, int file, const pp::BamImage* im, uint64_t r0, uint64_t r1);
+// After pp_tok_add_files: 1 when file `file` was BAM, with where its load's time went (read, inflate and record walk on the host -
+// zero for a range of a caller's image - and the image with its record offsets to HBM); 0 for SAM text.
+int pp_tok_bam_phases(pp_ctx* ctx, int file, float* read_ms, float* inflate_ms, float* walk_ms, float* upload_ms);
 
 // `polypolish filter` with the SAM text handled on the device (tok_kernels.cu); what the log of pp_filter_files prints.
 struct pp_filter_file_stats {

@@ -463,6 +463,22 @@ extern "C" void pp_pack_free(pp_pack* p) { delete p; }
 
 extern "C" int pp_pack_add_sam_file(pp_pack* P, const char* path) {
     if (!P || !path) return PP_ERR_ARG;
+    if (pp::is_bam(path)) {
+        // A BAM file is parsed as its SAM text: the header text, then one line per record (bam.cpp), so that every rule and every
+        // message of the text path - line numbers included - holds for it unchanged.
+        std::string sam, err;
+        int rc = PP_OK;
+        {
+            pp::BamImage im;
+            rc = pp::bam_load(path, nullptr, im, err);
+            if (rc == PP_OK) rc = pp::bam_to_sam(im, sam, err);
+        }
+        if (rc != PP_OK) { P->error = err; P->error_code = rc; return rc; }
+        if (!P->replaying) P->sources.push_back({true, path, std::string()});
+        unsigned nt = P->threads ? P->threads : std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
+        return (nt > 1 && sam.size() >= 2 * P->min_chunk) ? pack_text_parallel(P, sam.data(), sam.size(), path, nt, P->min_chunk)
+                                                          : pack_text(P, sam.data(), sam.size(), path);
+    }
     // A big regular file is read by several threads, each pread()ing its slice straight into one buffer (one pass, the page faults of
     // the buffer spread over the threads); anything else - a small file, a pipe, a device - is read into a string.  (Not mmap: a
     // file that another process truncates while it is parsed would raise SIGBUS; a short read is simply handled.)

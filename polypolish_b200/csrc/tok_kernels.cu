@@ -14,6 +14,10 @@
 //   (cub scan)    read ids
 //   k_tok_groups  one thread per group head: SEQ="*" records take the group's source sequence
 //
+// A BAM file (bam.cpp: inflated on the host into one image with its record offsets) takes a second front end: the image goes up
+// through the same pinned slots, k_bam_parse (one thread per record, bam_rec.h) stands in for the three line passes and
+// k_bam_emit for k_tok_emit; the scans, k_tok_heads and k_tok_groups are shared.
+//
 // Per-item logic lives in tok_line.h (host+device, CPU-tested against the host packer).  The host packer stays the
 // authority on everything unusual: a malformed line, a limit, a group without sequence make the call return PP_TOK_HOST and
 // the caller runs pp_pack_* on the same text, which yields the result or the reference's own error message
@@ -42,6 +46,7 @@
 #include "tok_line.h"
 #include "tok_table.h"
 #include "tok_strip.h"
+#include "bam_rec.h"
 
 // A temporary that does not fit in device memory is not an error of the data: the host text code takes over.
 #define TRY_ALLOC(x) do { if ((x) != cudaSuccess) { cudaGetLastError(); return PP_TOK_HOST; } } while (0)
@@ -215,6 +220,54 @@ __global__ void __launch_bounds__(TK_LINE_THREADS) k_tok_groups(uint64_t n_al, c
     if (head[a] && !tok::close_group(a, n_al, head, careful != 0, seq_off, seq_len, flags)) st->group_err = 1;
 }
 
+// ---- BAM records (bam_rec.h): the image of the file stands in for the text, record offsets for line starts
+struct BamArgs {
+    ParseArgs p;
+    const uint32_t* ref_contig;       // [n_ref + 1]
+    uint32_t n_ref;
+};
+
+__global__ void __launch_bounds__(TK_LINE_THREADS) k_bam_parse(BamArgs a) {
+    const uint64_t i = (uint64_t)blockIdx.x * TK_LINE_THREADS + threadIdx.x;
+    if (i > a.p.n_lines) return;
+    if (i == a.p.n_lines) { a.p.s_al[i] = 0; a.p.s_ops[i] = 0; a.p.s_blk[i] = 0; return; }
+    tok::Txt x(a.p.text);
+    tok::LineRec r;
+    uint8_t fault;
+    const uint8_t kind = tok::parse_bam(x, a.p.line_start[i], a.ref_contig, a.n_ref, r, fault);
+    a.p.recs[i] = r;
+    const bool al = kind == tok::LK_ALIGNED;
+    a.p.s_al[i] = al ? 1 : 0;
+    a.p.s_ops[i] = al ? r.nops : 0;
+    a.p.s_blk[i] = al ? tok::seq_blocks(r) : 0;
+    if (kind == tok::LK_HOST) atomicMin(&a.p.st->first_bad, (unsigned long long)i);
+}
+
+template <int BITS>
+__global__ void __launch_bounds__(TK_LINE_THREADS) k_bam_emit(EmitArgs a) {
+    const uint64_t i = (uint64_t)blockIdx.x * TK_LINE_THREADS + threadIdx.x;
+    if (i >= a.p.n_lines) return;
+    const tok::LineRec r = a.p.recs[i];
+    if (r.kind != tok::LK_ALIGNED) return;
+    const uint64_t s = a.p.line_start[i];
+    const uint64_t la = a.p.s_al[i], A = a.aln_base + la;
+    const uint64_t co = a.ops_base + a.p.s_ops[i], bo = a.blk_base + a.p.s_blk[i];
+    const bool star = r.flags & PP_FLAG_SEQSTAR;
+    a.contig[A] = r.contig;
+    a.ref_start[A] = r.ref_start;
+    a.seq_off[A] = star ? 0u : (uint32_t)bo;
+    a.seq_len[A] = (uint16_t)r.slen;
+    a.cigar_off[A] = (uint32_t)co;
+    a.n_cigar[A] = (uint16_t)r.nops;
+    a.nm[A] = r.nm;
+    a.flags[A] = r.flags;
+    a.name_pos[la] = s + tok::BAM_FIXED;          // read_name: k_tok_heads compares QNAMEs in the image as it does in text
+    a.name_len[la] = r.name_len;
+    tok::Txt x(a.p.text);
+    tok::emit_bam_cigar(x, s, r, a.cigar_ops + co);
+    if (tok::emit_bam_seq<BITS>(x, s, r, a.seq_pool + bo * (BITS == 4 ? 16 : 32))) a.p.st->need8 = 1;
+}
+
 }  // namespace
 
 struct TokFilterBufs;
@@ -262,6 +315,13 @@ struct TokState {
     std::vector<uint64_t> range_off, range_len;
     struct Mark { uint64_t aln, ops, blk, reads; };
     std::vector<Mark> marks;
+    // pp_tok_set_bam_range: file f of pp_tok_add_files is records [r0, r1) of an image the caller decoded (several contexts share it)
+    struct BamIn { const pp::BamImage* im = nullptr; uint64_t r0 = 0, r1 = 0; };
+    std::vector<BamIn> bam_in;
+    // what the last pp_tok_add_files found per file: BAM or not, and for a BAM where the load's time went (host read, inflate and
+    // record walk of bam.cpp - zero for an image the caller decoded - then the image and record offsets to HBM)
+    struct BamPhase { bool bam = false; float read_ms = 0, inflate_ms = 0, walk_ms = 0, upload_ms = 0; };
+    std::vector<BamPhase> phases;
     struct XState;                    // buffers of pp_tok_exchange_finish, kept between calls (no cudaMalloc in the steady state)
     XState* xs = nullptr;
     // pp_tok_set_shard: this context keeps one shard of the assembly
@@ -359,6 +419,15 @@ extern "C" int pp_tok_begin(pp_ctx* ctx, const pp_fasta* fa, int careful, int se
     T->shard_on = false;
     T->ranges_on = false;
     T->marks.clear();
+    T->bam_in.clear();
+    return PP_OK;
+}
+
+int pp_tok_set_bam_range(pp_ctx* ctx, int file, const pp::BamImage* im, uint64_t r0, uint64_t r1) {
+    TokState* T = ctx ? ctx->tok : nullptr;
+    if (!T || !T->active || file < 0 || !im || r0 > r1 || r1 > im->rec.size()) return PP_ERR_ARG;
+    if (T->bam_in.size() <= (size_t)file) T->bam_in.resize((size_t)file + 1);
+    T->bam_in[(size_t)file] = {im, r0, r1};
     return PP_OK;
 }
 
@@ -409,52 +478,33 @@ extern "C" int pp_tok_set_shard(pp_ctx* ctx, const uint32_t* local_of, uint32_t 
     return PP_OK;
 }
 
-// The text is on the device (n bytes, zero padded).  Appends its alignments to the dataset under construction.
-static int tok_process(pp_ctx* ctx, TokState* T, const uint8_t* text, uint64_t n, bool unterminated, pp_tok_stats* stats, bool part_of_file = false) {
-    cudaStream_t s = ctx->stream;
-    uint32_t launches = 0;
-    CK(cudaEventRecord(ctx->ev[0], s));
-    // ---- lines
-    const uint64_t n16 = (n + 15) & ~15ull;
-    const uint64_t n_tiles = (n16 + TK_TILE - 1) / TK_TILE;
-    if (n_tiles >= 0x7FFFFFFFull) return PP_TOK_HOST;
-    size_t cub_bytes = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, cub_bytes, (unsigned long long*)nullptr, (unsigned long long*)nullptr, (int64_t)std::max<uint64_t>(n_tiles + 1, 1)));
-    CK(T->cub.ensure(cub_bytes + 256));
-    TRY_ALLOC(ctx->b[B_TOKLINE].ensure((n_tiles + 2) * 8));
-    unsigned long long* tile_cnt = ctx->b[B_TOKLINE].as<unsigned long long>();
-    uint64_t n_lines = 0;
-    if (n_tiles) {
-        CK(cudaMemsetAsync(tile_cnt + n_tiles, 0, 8, s));
-        k_tok_count<<<(unsigned)n_tiles, TK_THREADS, 0, s>>>(text, n16, tile_cnt);
-        size_t tb = T->cub.cap;
-        CK(cub::DeviceScan::ExclusiveSum(T->cub.p, tb, tile_cnt, tile_cnt, (int64_t)(n_tiles + 1), s));
-        CK(cudaMemcpyAsync(T->h_tot, tile_cnt + n_tiles, 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        launches += 3;
-        n_lines = T->h_tot[0] + (unterminated ? 1 : 0);
-    }
-    if (stats) stats->lines = n_lines;
-    if (n_lines == 0) return part_of_file ? PP_OK : PP_TOK_HOST;   // "no alignments in <file>": the host packer words it (a byte range may be empty)
-    if (n_lines >= 0xFFFFFFF0ull) return PP_TOK_HOST;
-
-    // scratch: line starts | line records | three scan arrays
+// Scratch of the per-line passes (one line = one SAM text line or one BAM record): line starts | line records | three scan arrays;
+// the status is reset.
+static int line_scratch(pp_ctx* ctx, TokState* T, const uint8_t* text, uint64_t n, uint64_t n_lines, ParseArgs& pa) {
     size_t off = 0;
     auto carve = [&](size_t bytes) { size_t o = off; off += (bytes + 255) & ~size_t(255); return o; };
     const size_t o_ls = carve((n_lines + 2) * 8), o_rec = carve(n_lines * sizeof(tok::LineRec)), o_al = carve((n_lines + 1) * 8),
                  o_ops = carve((n_lines + 1) * 8), o_blk = carve((n_lines + 1) * 8);
     TRY_ALLOC(ctx->b[B_TOKTMP].ensure(off));
     uint8_t* tmp = ctx->b[B_TOKTMP].as<uint8_t>();
-    ParseArgs pa;
-    pa.text = text; pa.n = n; pa.line_start = (unsigned long long*)(tmp + o_ls); pa.n_lines = n_lines; pa.unterminated = unterminated ? 1 : 0;
+    pa.text = text; pa.n = n; pa.line_start = (unsigned long long*)(tmp + o_ls); pa.n_lines = n_lines; pa.unterminated = 0;
     pa.tb = T->tb; pa.recs = (tok::LineRec*)(tmp + o_rec);
     pa.s_al = (unsigned long long*)(tmp + o_al); pa.s_ops = (unsigned long long*)(tmp + o_ops); pa.s_blk = (unsigned long long*)(tmp + o_blk);
     pa.st = T->d_st;
     T->h_st->first_bad = ~0ull; T->h_st->need8 = 0; T->h_st->group_err = 0;
-    CK(cudaMemcpyAsync(T->d_st, T->h_st, sizeof(TokStatus), cudaMemcpyHostToDevice, s));
-    k_tok_index<<<(unsigned)n_tiles, TK_THREADS, 0, s>>>(text, n16, tile_cnt, (unsigned long long*)(tmp + o_ls));
-    const unsigned line_grid = (unsigned)((n_lines + 1 + TK_LINE_THREADS - 1) / TK_LINE_THREADS);
-    k_tok_parse<<<line_grid, TK_LINE_THREADS, 0, s>>>(pa);
+    CK(cudaMemcpyAsync(T->d_st, T->h_st, sizeof(TokStatus), cudaMemcpyHostToDevice, ctx->stream));
+    return PP_OK;
+}
+
+// What the SAM and the BAM front ends share once the parse pass has run: the scans (alignment index, CIGAR-pool and sequence-pool
+// offsets), the dataset arrays, the emit pass (`emit(ea, grid)` launches the front end's emit kernel), read groups, the SEQ="*"
+// sources, and the commit of the dataset bases.
+template <class Emit>
+static int tok_emit_groups(pp_ctx* ctx, TokState* T, const ParseArgs& pa, bool part_of_file, uint32_t launches, pp_tok_stats* stats, Emit&& emit) {
+    cudaStream_t s = ctx->stream;
+    const uint8_t* text = pa.text;
+    const uint64_t n = pa.n, n_lines = pa.n_lines;
+    size_t cub_bytes = 0;
     CK(cub::DeviceScan::ExclusiveSum(nullptr, cub_bytes, pa.s_al, pa.s_al, (int64_t)(n_lines + 1)));
     CK(T->cub.ensure(cub_bytes + 256));
     for (unsigned long long* arr : {pa.s_al, pa.s_ops, pa.s_blk}) {
@@ -466,7 +516,7 @@ static int tok_process(pp_ctx* ctx, TokState* T, const uint8_t* text, uint64_t n
     CK(cudaMemcpyAsync(T->h_tot + 2, pa.s_blk + n_lines, 8, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(T->h_st, T->d_st, sizeof(TokStatus), cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
-    launches += 5;
+    launches += 3;
     const uint64_t n_al = T->h_tot[0], n_ops = T->h_tot[1], n_blk = T->h_tot[2];
     if (stats) stats->alignments = n_al;
     if (T->h_st->first_bad != ~0ull) return PP_TOK_HOST;
@@ -502,9 +552,7 @@ static int tok_process(pp_ctx* ctx, TokState* T, const uint8_t* text, uint64_t n
     ea.seq_len = ctx->b[B_SEQLEN].as<uint16_t>(); ea.n_cigar = ctx->b[B_NCIG].as<uint16_t>();
     ea.flags = ctx->b[B_FLAGS].as<uint8_t>(); ea.seq_pool = ctx->b[B_SEQPOOL].as<uint8_t>();
     ea.name_pos = (unsigned long long*)(sc + o_np); ea.name_len = (uint32_t*)(sc + o_nl);
-    const unsigned emit_grid = (unsigned)((n_lines + TK_LINE_THREADS - 1) / TK_LINE_THREADS);
-    if (T->seq_bits == 4) k_tok_emit<4><<<emit_grid, TK_LINE_THREADS, 0, s>>>(ea);
-    else k_tok_emit<8><<<emit_grid, TK_LINE_THREADS, 0, s>>>(ea);
+    emit(ea, (unsigned)((n_lines + TK_LINE_THREADS - 1) / TK_LINE_THREADS));
     uint32_t* head = (uint32_t*)(sc + o_hd);
     uint32_t* rs = (uint32_t*)(sc + o_rs);
     const unsigned aln_grid = (unsigned)((n_al + TK_LINE_THREADS - 1) / TK_LINE_THREADS);
@@ -539,6 +587,50 @@ static int tok_process(pp_ctx* ctx, TokState* T, const uint8_t* text, uint64_t n
     return PP_OK;
 }
 
+
+// The text is on the device (n bytes, zero padded).  Appends its alignments to the dataset under construction.
+static int tok_process(pp_ctx* ctx, TokState* T, const uint8_t* text, uint64_t n, bool unterminated, pp_tok_stats* stats, bool part_of_file = false) {
+    cudaStream_t s = ctx->stream;
+    uint32_t launches = 0;
+    CK(cudaEventRecord(ctx->ev[0], s));
+    // ---- lines
+    const uint64_t n16 = (n + 15) & ~15ull;
+    const uint64_t n_tiles = (n16 + TK_TILE - 1) / TK_TILE;
+    if (n_tiles >= 0x7FFFFFFFull) return PP_TOK_HOST;
+    size_t cub_bytes = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, cub_bytes, (unsigned long long*)nullptr, (unsigned long long*)nullptr, (int64_t)std::max<uint64_t>(n_tiles + 1, 1)));
+    CK(T->cub.ensure(cub_bytes + 256));
+    TRY_ALLOC(ctx->b[B_TOKLINE].ensure((n_tiles + 2) * 8));
+    unsigned long long* tile_cnt = ctx->b[B_TOKLINE].as<unsigned long long>();
+    uint64_t n_lines = 0;
+    if (n_tiles) {
+        CK(cudaMemsetAsync(tile_cnt + n_tiles, 0, 8, s));
+        k_tok_count<<<(unsigned)n_tiles, TK_THREADS, 0, s>>>(text, n16, tile_cnt);
+        size_t tb = T->cub.cap;
+        CK(cub::DeviceScan::ExclusiveSum(T->cub.p, tb, tile_cnt, tile_cnt, (int64_t)(n_tiles + 1), s));
+        CK(cudaMemcpyAsync(T->h_tot, tile_cnt + n_tiles, 8, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        launches += 3;
+        n_lines = T->h_tot[0] + (unterminated ? 1 : 0);
+    }
+    if (stats) stats->lines = n_lines;
+    if (n_lines == 0) return part_of_file ? PP_OK : PP_TOK_HOST;   // "no alignments in <file>": the host packer words it (a byte range may be empty)
+    if (n_lines >= 0xFFFFFFF0ull) return PP_TOK_HOST;
+
+    ParseArgs pa;
+    int rc = line_scratch(ctx, T, text, n, n_lines, pa);
+    if (rc != PP_OK) return rc;
+    pa.unterminated = unterminated ? 1 : 0;
+    k_tok_index<<<(unsigned)n_tiles, TK_THREADS, 0, s>>>(text, n16, tile_cnt, const_cast<unsigned long long*>(pa.line_start));
+    const unsigned line_grid = (unsigned)((n_lines + 1 + TK_LINE_THREADS - 1) / TK_LINE_THREADS);
+    k_tok_parse<<<line_grid, TK_LINE_THREADS, 0, s>>>(pa);
+    launches += 2;
+    return tok_emit_groups(ctx, T, pa, part_of_file, launches, stats, [&](const EmitArgs& ea, unsigned grid) {
+        if (T->seq_bits == 4) k_tok_emit<4><<<grid, TK_LINE_THREADS, 0, s>>>(ea);
+        else k_tok_emit<8><<<grid, TK_LINE_THREADS, 0, s>>>(ea);
+    });
+}
+
 static int text_buffer(pp_ctx* ctx, DevBuf& tb, uint64_t n) {
     CK(tb.ensure(n + 64));
     const uint64_t n16 = (n + 15) & ~15ull;
@@ -571,7 +663,8 @@ extern "C" int pp_tok_add_text(pp_ctx* ctx, const char* text, size_t len, pp_tok
 // Streams a file into dst: T->readers host threads, each pread()s its slices into its two pinned slots and sends them on
 // its own stream, so that page-cache reads, pinned staging and PCIe overlap.  Runs on the caller's thread or on the
 // prefetch thread; touches neither ctx->err nor ctx->stream.  Returns PP_OK / PP_ERR_IO / PP_ERR_CUDA (+ *cuda_err).
-static int upload_file(int device, TokState* T, uint8_t* dst, int fd, uint64_t n, uint8_t* last_byte, int* cuda_err, uint64_t foff = 0) {
+static int upload_file(int device, TokState* T, uint8_t* dst, int fd, uint64_t n, uint8_t* last_byte, int* cuda_err, uint64_t foff = 0,
+                       const uint8_t* mem = nullptr /* the bytes are in host memory (a BAM image), not in fd */) {
     const int R = T->readers;
     const uint64_t n_slices = (n + TK_SLOT - 1) / TK_SLOT;
     std::atomic<int> err{0};           // 1 = read error, 2 = CUDA error
@@ -587,6 +680,7 @@ static int upload_file(int device, TokState* T, uint8_t* dst, int fd, uint64_t n
             }
             const uint64_t o = sl * TK_SLOT, len = std::min<uint64_t>(TK_SLOT, n - o);
             uint64_t got = 0;
+            if (mem) memcpy(T->pin[r][slot], mem + o, (size_t)len), got = len;
             while (got < len) {
                 const ssize_t g = pread(fd, T->pin[r][slot] + got, (size_t)(len - got), (off_t)(foff + o + got));
                 if (g <= 0) { err = 1; return; }
@@ -782,6 +876,7 @@ extern "C" int pp_tok_prefetch(pp_ctx* ctx, const char* path) {
     int rc = tok_state(ctx, &T);
     if (rc) return rc;
     if (T->pf.active) return PP_OK;                            // one outstanding upload at a time
+    if (pp::is_bam(path)) return PP_OK;                        // a BAM is inflated on the host first (tok_add_bam)
     rc = prefetch_start(ctx, T, path, true);
     return rc == PP_TOK_HOST ? PP_OK : rc;                     // pp_tok_add_file(s) will say so
 }
@@ -795,6 +890,65 @@ extern "C" int pp_tok_expect(pp_ctx* ctx, uint64_t total_text_bytes) {
     return PP_OK;
 }
 
+// Records [r0, r1) of a BAM image -> appended to the dataset under construction.  The image crosses PCIe through the reader slots,
+// then k_bam_parse / k_bam_emit decode it in place.  `next` (may be null): the next file, which starts streaming in once the slots
+// are free again (a SAM file: the caller has classified it).  host_ms: what reading, inflating and walking the file took (part of
+// h2d_ms); *upload_ms: the image and the record offsets to HBM.
+static int tok_add_bam(pp_ctx* ctx, TokState* T, const pp::BamImage& im, uint64_t r0, uint64_t r1, pp_tok_stats* stats, float host_ms,
+                       const char* next, int next_range, float* upload_ms) {
+    cudaStream_t s = ctx->stream;
+    const uint64_t n_rec = r1 - r0;
+    if (stats) stats->lines = n_rec;
+    if (!im.device_ok) return PP_TOK_HOST;
+    if (n_rec == 0) return T->ranges_on ? PP_OK : PP_TOK_HOST;         // "no alignments in <file>": the host packer words it
+    if (n_rec >= 0xFFFFFFF0ull) return PP_TOK_HOST;
+    const uint64_t b0 = im.rec[r0], b1 = r1 < im.rec.size() ? im.rec[r1] : im.size, n = b1 - b0;
+    int rc = ring_ready(ctx, T);
+    if (rc != PP_OK) return rc;
+    const int buf = T->next_buf;
+    T->next_buf ^= 1;
+    DevBuf& tb = T->text[buf];
+    if (tb.cap < n + 64) {                                             // the same room as a SAM text of this size needs
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || (double)free_b + (double)tb.cap < 2.6 * (double)n + (256 << 20)) {
+            cudaGetLastError();
+            return PP_TOK_HOST;
+        }
+    }
+    rc = text_buffer(ctx, tb, n);
+    if (rc != PP_OK) { cudaGetLastError(); return PP_TOK_HOST; }
+    const auto t0 = std::chrono::steady_clock::now();
+    uint8_t last = 0;
+    int cerr = 0;
+    rc = upload_file(ctx->device, T, tb.as<uint8_t>(), -1, n, &last, &cerr, 0, im.data.p + b0);
+    if (rc == PP_ERR_CUDA) return ctx->fail_cuda((cudaError_t)cerr, "BAM image upload", __FILE__, __LINE__);
+    ParseArgs pa;
+    if ((rc = line_scratch(ctx, T, tb.as<uint8_t>(), n, n_rec, pa)) != PP_OK) return rc;
+    {
+        std::vector<unsigned long long> off((size_t)n_rec);
+        for (uint64_t k = 0; k < n_rec; ++k) off[(size_t)k] = im.rec[r0 + k] - b0;
+        CK(cudaMemcpyAsync(const_cast<unsigned long long*>(pa.line_start), off.data(), (size_t)n_rec * 8, cudaMemcpyHostToDevice, s));
+        TRY_ALLOC(ctx->b[B_TOKLINE].ensure(im.ref_contig.size() * 4 + 16));
+        CK(cudaMemcpyAsync(ctx->b[B_TOKLINE].p, im.ref_contig.data(), im.ref_contig.size() * 4, cudaMemcpyHostToDevice, s));
+        CK(cudaStreamSynchronize(s));                                   // (pageable sources)
+    }
+    *upload_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    const float h2d = host_ms + *upload_ms;
+    if (next && (rc = prefetch_start(ctx, T, next, true, next_range)) < 0) return rc;
+    CK(cudaEventRecord(ctx->ev[0], s));
+    BamArgs ba;
+    ba.p = pa;
+    ba.ref_contig = ctx->b[B_TOKLINE].as<uint32_t>();
+    ba.n_ref = (uint32_t)im.ref_names.size();
+    k_bam_parse<<<(unsigned)((n_rec + 1 + TK_LINE_THREADS - 1) / TK_LINE_THREADS), TK_LINE_THREADS, 0, s>>>(ba);
+    rc = tok_emit_groups(ctx, T, pa, T->ranges_on, 1, stats, [&](const EmitArgs& ea, unsigned grid) {
+        if (T->seq_bits == 4) k_bam_emit<4><<<grid, TK_LINE_THREADS, 0, s>>>(ea);
+        else k_bam_emit<8><<<grid, TK_LINE_THREADS, 0, s>>>(ea);
+    });
+    if (stats) { stats->h2d_ms = h2d; stats->h2d_bytes = n + n_rec * 8; }
+    return rc;
+}
+
 extern "C" int pp_tok_add_files(pp_ctx* ctx, const char* const* paths, int n_paths, pp_tok_stats* stats) {
     if (!ctx) return PP_ERR_ARG;
     TokState* T = ctx->tok;
@@ -804,9 +958,31 @@ extern "C" int pp_tok_add_files(pp_ctx* ctx, const char* const* paths, int n_pat
     if (stats) memset(stats, 0, sizeof(pp_tok_stats) * (size_t)n_paths);
     if (T->ranges_on && T->range_off.size() != (size_t)n_paths) return ctx->fail(PP_ERR_ARG, "pp_tok_add_files: as many paths as pp_tok_set_ranges ranges");
     const bool ranges = T->ranges_on;
+    // every input is classified once, here: a range of an image the caller decoded, a BAM file, or SAM text
+    T->phases.assign((size_t)n_paths, TokState::BamPhase());
     for (int i = 0; i < n_paths; ++i) {
         if (!paths[i]) return ctx->fail(PP_ERR_ARG, "pp_tok_add_file: null path");
+        T->phases[(size_t)i].bam = ((size_t)i < T->bam_in.size() && T->bam_in[(size_t)i].im) || pp::is_bam(paths[i]);
+    }
+    auto is_sam = [&](int j) { return j < n_paths && !T->phases[(size_t)j].bam; };
+    for (int i = 0; i < n_paths; ++i) {
         T->marks.push_back({T->aln_base, T->ops_base, T->blk_base, T->read_base});
+        TokState::BamPhase& ph = T->phases[(size_t)i];
+        const TokState::BamIn* shared = (size_t)i < T->bam_in.size() && T->bam_in[(size_t)i].im ? &T->bam_in[(size_t)i] : nullptr;
+        if (ph.bam) {
+            if (T->pf.active) { if (T->pf.th.joinable()) T->pf.th.join(); T->pf.active = false; }   // (the reader slots are needed)
+            if (!shared && ranges) { T->active = false; return PP_TOK_HOST; }                      // byte ranges are SAM-only
+            pp::BamImage own;
+            std::string err;
+            if (!shared && pp::bam_load(paths[i], T->fasta, own, err) != PP_OK) { T->active = false; return PP_TOK_HOST; }   // the host words it
+            const pp::BamImage& im = shared ? *shared->im : own;
+            if (!shared) { ph.read_ms = im.read_ms; ph.inflate_ms = im.inflate_ms; ph.walk_ms = im.walk_ms; }
+            const char* next = is_sam(i + 1) ? paths[i + 1] : nullptr;
+            const int brc = tok_add_bam(ctx, T, im, shared ? shared->r0 : 0, shared ? shared->r1 : im.rec.size(), stats ? stats + i : nullptr,
+                                        ph.read_ms + ph.inflate_ms + ph.walk_ms, next, ranges ? i + 1 : -1, &ph.upload_ms);
+            if (brc != PP_OK) { T->active = false; return brc; }
+            continue;
+        }
         int rc = prefetch_wait(ctx, T, paths[i], true, ranges ? i : -1);
         if (rc != PP_OK) { T->active = false; return rc; }
         const int buf = T->pf.buf;
@@ -814,7 +990,7 @@ extern "C" int pp_tok_add_files(pp_ctx* ctx, const char* const* paths, int n_pat
         const bool unterminated = n > 0 && T->pf.last != '\n';
         const float h2d = T->pf.ms;
         const uint64_t h2d_bytes = T->pf.sent;
-        if (i + 1 < n_paths && paths[i + 1]) {                 // the next file streams in while this one is tokenised
+        if (is_sam(i + 1)) {                                    // the next file streams in while this one is tokenised
             rc = prefetch_start(ctx, T, paths[i + 1], true, ranges ? i + 1 : -1);
             if (rc < 0) { T->active = false; return rc; }
         }
@@ -824,6 +1000,14 @@ extern "C" int pp_tok_add_files(pp_ctx* ctx, const char* const* paths, int n_pat
     }
     T->marks.push_back({T->aln_base, T->ops_base, T->blk_base, T->read_base});
     return PP_OK;
+}
+
+int pp_tok_bam_phases(pp_ctx* ctx, int file, float* read_ms, float* inflate_ms, float* walk_ms, float* upload_ms) {
+    TokState* T = ctx ? ctx->tok : nullptr;
+    if (!T || file < 0 || (size_t)file >= T->phases.size() || !T->phases[(size_t)file].bam) return 0;
+    const TokState::BamPhase& ph = T->phases[(size_t)file];
+    *read_ms = ph.read_ms; *inflate_ms = ph.inflate_ms; *walk_ms = ph.walk_ms; *upload_ms = ph.upload_ms;
+    return 1;
 }
 
 extern "C" int pp_tok_add_file(pp_ctx* ctx, const char* path, pp_tok_stats* stats) {
