@@ -1,6 +1,8 @@
 """The polish kernels themselves (k_prep -> stable sort -> k_bin_bounds -> k_tile -> k_compact, polypolish_b200/csrc/polish_dev.cuh)
 run on the CPU through tests/emu (one OS thread per CUDA thread) against the oracle, byte for byte.  This is a logic check of
-the device code for runs without a GPU; the real parity tests are the `-m gpu` ones.  PP_EMU_ALL=1 runs every fuzz seed."""
+the device code for runs without a GPU; the real parity tests are the `-m gpu` ones.  PP_EMU_ALL=1 runs every fuzz seed.  The fallback
+and boundary paths (long reads, queue overflow, global-k, node-pool and output overflow, long alleles, many contigs) are
+tests/test_emu_polish_limits.py, and on the device tests/test_gpu_polish_limits.py."""
 import os
 
 import pytest
